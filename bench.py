@@ -280,6 +280,27 @@ def parity_gate(O, eng, pages: np.ndarray, u, l, put_lens, threads: int) -> dict
     return O.parity_records(pages, u, l, recs, rec_lens, put_lens, ACCEL, threads)
 
 
+def dump_outputs(out_dir: str, eng, u, l, lens) -> None:
+    """Writes what the put path returned and stored for the last timed device-resident step: the
+    stored block length of every chunk, its 128-bit fingerprint (four 32-bit limbs), and the LZ4
+    blocks of a fixed, seeded sample of 64 chunks (byte values, -1 past the block's end).  The
+    pages are a function of the chunk ids and SEED alone, so two builds can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    fps, ok = eng.read_fingerprints(u, l)
+    assert ok.all(), "a chunk of the last step has no fingerprint"
+    limbs = np.stack([fps[:, 0] >> np.uint64(32), fps[:, 0] & np.uint64(0xFFFFFFFF),
+                      fps[:, 1] >> np.uint64(32), fps[:, 1] & np.uint64(0xFFFFFFFF)], axis=1)
+    pick = np.sort(np.random.default_rng(SEED).choice(len(u), size=min(64, len(u)), replace=False))
+    recs, rec_lens = eng.read_records_raw(u[pick], l[pick])
+    blocks = np.full((len(pick), recs.shape[1] - 24), -1.0, dtype=np.float32)
+    for i, n in enumerate(rec_lens):
+        blocks[i, :max(0, n - 24)] = recs[i, 24:n]
+    np.save(os.path.join(out_dir, "stored_lengths.npy"), np.asarray(lens, dtype=np.float64))
+    np.save(os.path.join(out_dir, "fingerprints.npy"), limbs.astype(np.float64))
+    np.save(os.path.join(out_dir, "block_sample_chunks.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "block_sample.npy"), blocks)
+
+
 def run_config_2_3(args, E, O, torch, local, d_pages, h_ptr, h_pages, peak, threads):
     """BASELINE configs 2 and 3 on this GPU (SURVEY.md §8d): a stream with 50 % same-address
     duplicates through put (key table insert / overwrite in place), then the read-hit path over
@@ -647,6 +668,8 @@ def run_ours(args):
     parity["what"] = ("records of the last device-resident step read back from the arena (cmb200_read_records) and its reported "
                       "stored lengths vs LZ4_compress_fast(accel 12) + data_prefix of the same pages")
     assert parity["mismatches"] == 0, f"parity gate failed: {parity}"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, u_last, l_last, lens)
 
     # ---- roofline of the dominant kernel (k_encode) ----
     peak, peak_src = peaks()
@@ -745,7 +768,11 @@ def main():
     ap.add_argument("--c4-steps", type=int, default=3)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    "(rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -101,3 +101,17 @@ def codec_cases():
     for cid in range(8):
         cases.append(("S", 65536, 12, cid))
     return cases
+
+
+# The cases that the oracle and the CUDA encoder are compared on with the compiled reference
+# (tests/golden/reference_lz4.json holds the reference's answers): (kind, nbytes, accel, seed).
+def reference_lz4_cases():
+    return [(kind, n, accel, 10_000 * rep + n + accel + ord(kind))
+            for rep in range(2)
+            for n in (4096, 16384, 65536, 131072, 65546, 65547, 13, 12, 1, 777)
+            for accel in (12, 1, 0, 5, 200)
+            for kind in "RTZMPAX"]
+
+
+def reference_cuda_cases():
+    return [("RTZMPAX"[i % 7], bs, 12, 9000 + i) for bs, n in ((65536, 84), (4096, 140)) for i in range(n)]

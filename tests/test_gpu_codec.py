@@ -240,14 +240,20 @@ print("plain-path parity ok")
 def test_cuda_blocks_equal_the_compiled_reference_directly(E, gpu, oracle):
     """CUDA == reference without the port in between: blocks and lengths of the GPU encoder against
     LZ4_compress_fast of oracle/_ref (the reference's own lz4.c compiled by oracle/Makefile), every
-    content class, 64 KiB and 4 KiB pages, and the reference's LZ4_decompress_fast decodes them back."""
-    if oracle.ref() is None:
-        pytest.skip("oracle/_ref was not built (needs /root/reference in the authoring container)")
-    for bs, n in ((65536, 84), (4096, 140)):
-        pages = np.stack([datagen.make_page("RTZMPAX"[i % 7], bs, 9000 + i) for i in range(n)])
+    content class, 64 KiB and 4 KiB pages, and the reference's LZ4_decompress_fast decodes them back.
+    Without oracle/_ref the reference's blocks stored in golden/reference_lz4.json (each of which
+    its decoder took back when they were recorded) stand in for it."""
+    gold = json.load(open(os.path.join(GOLD, "reference_lz4.json")))["cuda_cases"]
+    cases = datagen.reference_cuda_cases()
+    assert [tuple(c[:4]) for c in gold] == cases and len(cases) == 224
+    for bs in (65536, 4096):
+        idx = [j for j, c in enumerate(cases) if c[1] == bs]
+        pages = np.stack([datagen.make_page(kind, bs, seed) for kind, _, _, seed in (cases[j] for j in idx)])
         blocks, _ = E.lz4_encode_batch(pages, accel=12)
-        for i in range(n):
-            want = oracle.ref_lz4_encode(pages[i], 12)
-            assert blocks[i] == want, (bs, i)
-            back, used = oracle.ref_lz4_decode(want, bs)
-            assert used == len(want) and back == pages[i].tobytes()
+        for i, j in enumerate(idx):
+            assert len(blocks[i]) == gold[j][4] and sha(blocks[i]) == gold[j][5], (bs, i)
+            if oracle.ref() is not None:
+                want = oracle.ref_lz4_encode(pages[i], 12)
+                assert blocks[i] == want, (bs, i)
+                back, used = oracle.ref_lz4_decode(want, bs)
+                assert used == len(want) and back == pages[i].tobytes()

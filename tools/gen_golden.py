@@ -4,7 +4,10 @@
 own uint128.h).  Run in the authoring container only; the fixtures it writes are committed and
 are what pins the oracle (and, on the GPU box, the CUDA path) where /root/reference is absent.
 
-    python tools/gen_golden.py
+    python tools/gen_golden.py [lz4 keys reference exerciser store]     (default: all of them)
+
+`reference` and `exerciser` write the fixtures that stand in for the compiled reference in the tests
+that compare with it live (reference_lz4.json, reference_records.json; reference_exerciser.json).
 """
 from __future__ import annotations
 
@@ -133,9 +136,140 @@ def gen_store():
     os._exit(0)
 
 
+def _write(name, data):
+    with open(os.path.join(GOLD, name), "w") as f:
+        json.dump(data, f, indent=0)
+
+
+def gen_reference_lz4():
+    """The reference's blocks for the cases that test_oracle_vs_reference_live and
+    test_cuda_blocks_equal_the_compiled_reference_directly compare with."""
+    def case(kind, n, accel, seed):
+        page = datagen.make_page(kind, n, seed)
+        blk = O.ref_lz4_encode(page, accel)
+        back, used = O.ref_lz4_decode(blk, n)
+        assert back == page.tobytes() and used == len(blk)
+        return [kind, n, accel, seed, len(blk), sha(blk)]
+    _write("reference_lz4.json", {
+        "generator": "tools/gen_golden.py reference: LZ4_compress_fast of cachemap/lz4.c; every block decodes "
+                     "back with its LZ4_decompress_fast",
+        "version": O.ref().LZ4_versionString().decode(),
+        "oracle_cases": [case(*c) for c in datagen.reference_lz4_cases()],
+        "cuda_cases": [case(*c) for c in datagen.reference_cuda_cases()]})
+    print("reference lz4 cases written")
+
+
+def _ref_child(body: str):
+    """Runs `body` in a child with R = the compiled reference, under a watchdog: its cachemap_create
+    starts the put threads before it initialises their mutex and condition variable
+    (cachemap.c:123-138), and a child that loses that race never gets going."""
+    code = ("import sys, ctypes as C, numpy as np\n"
+            f"sys.path.insert(0, {ROOT!r}); sys.path.insert(0, {os.path.join(ROOT, 'tests')!r})\n"
+            "import datagen\nfrom oracle import ef_oracle as O\nR = O.ref()\n" + body +
+            "\nprint('child ok', flush=True)\nimport os; os._exit(0)\n")
+    for _ in range(6):
+        try:
+            r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120)
+        except subprocess.TimeoutExpired:
+            continue
+        assert r.returncode == 0 and "child ok" in r.stdout, r.stdout + r.stderr
+        return
+    raise RuntimeError("the reference library hung at start-up in every attempt")
+
+
+def _lmdb_records(exe, d, tmp):
+    """{(u, l): sha256 of the LMDB value without its 4 unspecified pad bytes} of a reference directory."""
+    from oracle import snapshot as S
+    snap = os.path.join(tmp, "from.snap")
+    subprocess.run([exe, "from-lmdb", d, snap, "16"], check=True, capture_output=True)
+    pshift, flags, recs = S.read_snapshot(snap)
+    assert pshift == 16 and flags == 0 and all(ts > 0 for ts, _, _, _ in recs)
+    out = {}
+    for _, _, _, rec in recs:
+        u, l = np.frombuffer(rec[:16], dtype=np.uint64)
+        out[(int(u), int(l))] = sha(rec[:20] + rec[24:])
+    return out
+
+
+def gen_reference_records():
+    """The records the reference keeps in its LMDB files for the puts of
+    test_snapshot_lmdb_interchange_on_the_reference_side and
+    test_cache_directory_interchange_with_the_reference, read back through tools/snap2lmdb."""
+    import pathlib
+    from test_oracle_pin import _build_snap2lmdb
+    with tempfile.TemporaryDirectory() as tmp:
+        exe = _build_snap2lmdb(pathlib.Path(tmp))
+        dirs = {k: os.path.join(tmp, k) for k in ("roundtrip", "gpu_to_ref", "ref_to_gpu")}
+        for d in dirs.values():
+            os.mkdir(d)
+        _ref_child(f"pages = O.gen_chunks(42, np.arange(24, dtype=np.uint64), 65536, 2)\n"
+                   f"cm = R.cachemap_create({dirs['roundtrip']!r}.encode(), 2048, 12, 16)\n"
+                   "for i in range(24):\n"
+                   "    R.cachemap_put(cm, i << 16, 777, 3, pages[i].ctypes.data)\n")
+        pages = "pages = np.stack([datagen.make_page('RTZMPAX'[i % 7], 65536, 300 + i) for i in range(48)])\n"
+        _ref_child(pages + f"cm = R.cachemap_create({dirs['gpu_to_ref']!r}.encode(), 2048, 12, 16)\n"
+                   "for i in range(48):\n"
+                   "    R.cachemap_put(cm, i << 16, 4242, 5, pages[i].ctypes.data)\n")
+        _ref_child(pages + f"cm = R.cachemap_create({dirs['ref_to_gpu']!r}.encode(), 2048, 12, 16)\n"
+                   "for i in range(48):\n"
+                   "    R.cachemap_put(cm, i << 16, 99, 7, pages[47 - i].ctypes.data)\n")
+        rt = _lmdb_records(exe, dirs["roundtrip"], tmp)
+        g2r = _lmdb_records(exe, dirs["gpu_to_ref"], tmp)
+        r2g = _lmdb_records(exe, dirs["ref_to_gpu"], tmp)
+    assert len(rt) == 24 and len(g2r) == 48 and len(r2g) == 48
+    _write("reference_records.json", {
+        "generator": "tools/gen_golden.py reference: cachemap_put of the compiled reference, its LMDB files read back "
+                     "with tools/snap2lmdb from-lmdb; sha256 of each value without its 4 unspecified pad bytes",
+        "roundtrip": sorted(rt.values()),
+        "gpu_to_ref": [g2r[(4242, (5 << 44) | i)] for i in range(48)],
+        "ref_to_gpu": [r2g[(99, (7 << 44) | i)] for i in range(48)]})
+    print("reference records written")
+
+
+def gen_reference_exerciser():
+    """Per-phase hits of tests/c/exerciser.c linked against the compiled reference.  One seed: most
+    starts of the reference lose its start-up race on a small host (see _ref_child)."""
+    import re
+    ref = os.path.join(ROOT, "oracle", "_ref", "libcachemap_ref.so")
+    runs = []
+    with tempfile.TemporaryDirectory() as tmp:
+        exe = os.path.join(tmp, "exer_ref")
+        subprocess.run(["gcc", "-O2", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "c", "exerciser.c"),
+                        "-o", exe, ref, f"-Wl,-rpath,{os.path.dirname(ref)}", "-lpthread"], check=True)
+        for seed in (1,):
+            out = None
+            for _ in range(12):
+                with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as d:
+                    try:
+                        out = subprocess.run([exe, d, "32768", "15", str(seed)], capture_output=True, text=True,
+                                             timeout=150, check=True).stdout
+                        break
+                    except subprocess.TimeoutExpired:
+                        continue
+            assert out is not None, "the reference library hung at start-up in every attempt"
+            runs.append({"seed": seed,
+                         "hits": {m.group(1): [int(m.group(2)), int(m.group(3))]
+                                  for m in re.finditer(r"phase (\w+) hits (\d+) of (\d+)", out)},
+                         "entries": [int(x) for x in re.findall(r"entries_after_\w+ (\d+)", out)]})
+    _write("reference_exerciser.json", {
+        "generator": "tools/gen_golden.py reference: tests/c/exerciser.c linked against the compiled reference, "
+                     "32 768 objects of 32 KiB, LMDB on tmpfs",
+        "runs": runs})
+    print("reference exerciser runs:", runs)
+
+
 if __name__ == "__main__":
     assert O.ref() is not None, "oracle/_ref/libcachemap_ref.so missing: run make -C oracle"
     os.makedirs(GOLD, exist_ok=True)
-    gen_lz4()
-    gen_keys()
-    gen_store()
+    which = sys.argv[1:] or ["lz4", "keys", "reference", "exerciser", "store"]
+    if "lz4" in which:
+        gen_lz4()
+    if "keys" in which:
+        gen_keys()
+    if "reference" in which:
+        gen_reference_lz4()
+        gen_reference_records()
+    if "exerciser" in which:
+        gen_reference_exerciser()
+    if "store" in which:
+        gen_store()                                   # last: it ends the process (see gen_store)
